@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — denoise-step throughput of the StreamingSVD hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = ONE pass of the hot path over one batch: StreamingWrapper.forward (ControlNet on 2x7 frames + VideoUNet
 with 13 CAM mergers on 2x25 frames, 576x1024 -> latent 72x128, classifier-free-guidance batch 2) followed by the
@@ -411,6 +411,8 @@ def run_ours(args):
     launches = ops.launches() - l0
     ms = e0.elapsed_time(e1)
     finite = bool(torch.isfinite(cur).all())
+    # what the last timed step handed back: the sampler's next latent state
+    outputs = {"latent": cur.float().cpu().numpy()} if args.dump_outputs else None
 
     # ---------------- e2e leg: host buffers, H2D + D2H every step ----------------
     out_host = torch.empty((T, 4, h, w), dtype=torch.float32).pin_memory()
@@ -591,6 +593,11 @@ def run_ours(args):
                 line["cpu_baseline"] = cpu_reference_sample()
             except Exception as exc:  # the GPU number must not be lost to a host-side problem
                 line["cpu_baseline"] = {"error": repr(exc)}
+        if outputs is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -665,7 +672,11 @@ def main():
     ap.add_argument("--no-replicas-leg", action="store_true")
     ap.add_argument("--mode", default="latency", choices=["latency", "throughput"],
                     help="N>1 only: latency = guidance halves on rank pairs (default), throughput = N replicas")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32), for comparing builds")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -675,7 +686,8 @@ def main():
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",
                "--master-addr", "127.0.0.1", "--master-port", os.environ.get("MASTER_PORT", "29511"),
                os.path.abspath(__file__), "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup",
-               str(args.warmup), "--mode", args.mode] + (["--no-cpu-baseline"] if args.no_cpu_baseline else [])
+               str(args.warmup), "--mode", args.mode] + (["--no-cpu-baseline"] if args.no_cpu_baseline else []) + \
+              (["--dump-outputs", args.dump_outputs] if args.dump_outputs else [])
         raise SystemExit(subprocess.call(cmd))
     run_ours(args)
 

@@ -40,6 +40,9 @@ CASES = {
     # full width + APM (17 context tokens), 25 frames, extents that are not powers of two on any level
     "full_apm_t25_24x40": (dataclasses.replace(arch.UNetConfig(), use_apm=True), 25, 24, 40, 17, 22),
 }
+# every fixture stays under 1 MB: name -> (channel step of the stored ControlNet taps, latent-row step of the stored
+# output); the tests slice their own tensors likewise and check the whole output against the oracle
+SAMPLING = {"tiny_t7_24x40": (2, 1), "full_t8_64x64": (32, 2), "full_apm_t25_24x40": (8, 1)}
 
 
 def check_grammar(wrapper, cfg):
@@ -92,11 +95,11 @@ def run_case(name, cfg, T, h, w, ctx_tokens, seed):
     scale = ref_out.abs().max().item()
     assert err <= 2e-4 * max(scale, 1.0), f"oracle restatement deviates from the reference: {err}"
     os.makedirs(GOLDEN, exist_ok=True)
-    cstep = 8 if name.startswith("full") else 1
+    cstep, rstep = SAMPLING.get(name, (1, 1))
     np.savez_compressed(
         os.path.join(GOLDEN, f"streaming_{name}.npz"),
-        out=ref_out.numpy().astype(np.float32),
-        # full-width cases keep every 8th channel of the ControlNet taps (fixture size); the test slices likewise
+        out=ref_out[:, :, ::rstep].numpy().astype(np.float32),
+        out_rstep=np.array([rstep], np.int64),
         ctrl_mid=captured["mid"][:, ::cstep].numpy().astype(np.float32),
         ctrl_hs_last=captured["hs"][-1][:, ::cstep].numpy().astype(np.float32),
         ctrl_cstep=np.array([cstep], np.int64),

@@ -6,6 +6,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -35,6 +38,19 @@ def test_product_arm_needs_a_gpu():
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "3",
                         "--no-cpu-baseline"], capture_output=True, text=True, timeout=300, cwd=ROOT)
     assert p.returncode != 0 and "no CPU path" in (p.stderr + p.stdout)
+
+
+@pytest.mark.gpu
+def test_product_arm_dumps_its_last_step(cuda_dev, tmp_path):
+    """--dump-outputs writes what the last timed step returned (the sampler's next latent) as float32."""
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--settle", "0",
+                        "--no-cpu-baseline", "--no-gpu-reference", "--no-chunk", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert p.returncode == 0, p.stderr[-2000:]
+    d = json.loads([ln for ln in p.stdout.splitlines() if ln.strip()][-1])
+    assert d["steps"] == 2 and d["finite"]
+    z = np.load(tmp_path / "latent.npy")
+    assert z.dtype == np.float32 and z.shape == (25, 4, 72, 128) and np.isfinite(z).all()
 
 
 def test_usable_cores_respects_affinity():

@@ -37,6 +37,7 @@ def test_streaming_wrapper_vs_reference_golden(cuda_dev, name, apm):
     base = arch.UNetConfig() if name.startswith("full") else arch.TINY
     cfg = dataclasses.replace(base, use_apm=bool(use_apm))
     cstep = int(g["ctrl_cstep"][0]) if "ctrl_cstep" in g else 1
+    rstep = int(g["out_rstep"][0]) if "out_rstep" in g else 1         # latent rows kept of the output
     sd_u = arch.synth_state_dict(arch.unet_param_shapes(cfg), seed=seed)
     sd_c = arch.synth_state_dict(arch.controlnet_param_shapes(cfg), seed=seed + 1000)
     x, t, c, kw = synth.make_inputs(cfg, T=T, h=h, w=w, seed=seed, ctx_tokens=ctx_tokens)
@@ -50,8 +51,9 @@ def test_streaming_wrapper_vs_reference_golden(cuda_dev, name, apm):
     out = out.float().cpu()
     assert torch.isfinite(out).all()
     ref = torch.from_numpy(g["out"])
-    r = _rel(out, ref)
-    mx = (out - ref).abs().max().item()
+    assert out[:, :, ::rstep].shape == ref.shape
+    r = _rel(out[:, :, ::rstep], ref)
+    mx = (out[:, :, ::rstep] - ref).abs().max().item()
     print(f"[{name}] out vs REFERENCE golden: rel_l2={r:.4e} max_abs={mx:.4e} ref_absmax={ref.abs().max():.3f}")
     # second call (exercises the cached conditioning path) must reproduce the first bit for bit
     out2 = m(xd, td, cd, **kwd).float().cpu()
@@ -60,7 +62,9 @@ def test_streaming_wrapper_vs_reference_golden(cuda_dev, name, apm):
     taps = {}
     with torch.no_grad():
         o_ref = orc.streaming_wrapper_forward(sd_u, sd_c, cfg, x, t, c, taps=taps, **kw)
-    assert _rel(o_ref, ref) < 1e-4  # the oracle itself reproduces the reference's golden output
+    assert _rel(o_ref[:, :, ::rstep], ref) < 1e-4  # the oracle itself reproduces the reference's golden output
+    # so the whole output is held to the oracle with the golden's tolerance, rows the fixture does not store included
+    assert _rel(out, o_ref) < REL_TOL and (out - o_ref).abs().max().item() < 6e-2 * o_ref.abs().max().item()
     worst = 0.0
     for tname, (tt, n, hh, ww) in m.engine.debug_taps.items():
         if tname in taps:
